@@ -11,7 +11,10 @@ process so that the driver's records cover them:
   configs[3]  LMPC Monte-Carlo rollouts, 8192 controllers per GPU, device-resident closed loop, pooled safe-set exchange with
               one NCCL all-gather per lap (benchmarks/rollout_mc.py).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config 1|2|3]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config 1|2|3] [--dump-outputs DIR]
+
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step of configs[1] and configs[2] returned to its caller
+as DIR/config1_<name>.npy and DIR/config2_<name>.npy (float64; inputs are seeded, so two builds can be compared array by array).
 
 Under torchrun (N > 1) every rank owns its own batch on its own GPU (weak scaling; instances are independent — SURVEY §8e);
 timing is CUDA events on the launching stream, max over ranks.  `--impl reference` times the CPU oracle
@@ -24,6 +27,8 @@ import subprocess
 import sys
 import threading
 import time
+
+sys.dont_write_bytecode = True      # the tree may be read-only; nothing of a run is written into it
 
 # one OpenMP thread per physical core, pinned: the CPU arm has to be repeatable (set before the oracle library loads)
 os.environ.setdefault("OMP_PROC_BIND", "spread")
@@ -50,6 +55,7 @@ FLOPS_PER_ITER = 12 * 2 * (288 + 216 + 126 + 72 + 36 + 48) + 4 * 12 * 2 * 126 + 
 FLOPS_PER_ITER_LMPC = FLOPS_PER_ITER + 2 * 48 * (21 + 6 * 6) + 2000       # + simplex terminal block (W assembly, recoveries)
 # fp64 tensor-core instructions issued per iteration: 12 stages x (11 factor + 4 corrector gradient + 2 x 4 forward)
 DMMA_PER_ITER = 12 * (11 + 4 + 8) + 2 * 6 + 2 * 2     # sweeps per stage + stage-gradient / right-hand-side tiles of 8 stages
+DUMP_LIMIT = 60 * 10**6          # array bytes --dump-outputs writes at most: below 64 MB with the .npy headers
 
 
 def dist_env():
@@ -263,6 +269,23 @@ def _traffic(kernel):
         return None
 
 
+def dump_outputs(path, groups):
+    """--dump-outputs: every array of ``groups`` ({prefix: {name: array[B, ...]}}) as path/<prefix>_<name>.npy in float64.  Above
+    DUMP_LIMIT bytes in all, each group keeps the same fixed, seeded sample of its B instances (indices in <prefix>_sample_index.npy)."""
+    row_bytes = {p: 8 * (1 + sum(np.asarray(a)[0].size for a in g.values())) for p, g in groups.items()}
+    total = sum(row_bytes[p] * len(next(iter(g.values()))) for p, g in groups.items())
+    frac = min(1.0, DUMP_LIMIT / total)
+    os.makedirs(path, exist_ok=True)
+    for p, g in groups.items():
+        B = len(next(iter(g.values())))
+        idx = np.arange(B)
+        if frac < 1.0:
+            idx = np.sort(np.random.default_rng(0).choice(B, max(1, int(B * frac)), replace=False))
+            np.save(os.path.join(path, p + "_sample_index.npy"), idx.astype(np.float64))
+        for name, a in g.items():
+            np.save(os.path.join(path, "%s_%s.npy" % (p, name)), np.asarray(a)[idx].astype(np.float64))
+
+
 def _max_over_ranks(v, dev, world):
     import torch
     import torch.distributed as dist
@@ -341,6 +364,9 @@ def leg_config1(args, rank, world, local, dev):
     step_ms = [a.elapsed_time(b) for a, b in ev]
     total_ms = _max_over_ranks(sum(step_ms), dev, world)
     status, iters, resid = d_st.cpu().numpy(), d_it.cpu().numpy(), d_rs.cpu().numpy()
+    outputs = None
+    if args.dump_outputs:
+        outputs = dict(xPred=d_xP.cpu().numpy(), uPred=d_uP.cpu().numpy(), status=status, iters=iters, resid=resid)
     # nvidia-smi polling takes driver locks that stall cudaMemcpyAsync enqueues: the sampler covers the device-timed region
     # only and is stopped before the host-timed leg (measured: 2.6-3.4 M/s with it running, 3.9 M/s without)
     clocks = sampler.stop() if rank == 0 else None
@@ -377,17 +403,17 @@ def leg_config1(args, rank, world, local, dev):
     solver.close()
     return dict(B=B, total_ms=total_ms, step_ms=step_ms, launches=int(launches), status=status, iters=iters, resid=resid, clocks=clocks,
                 e2e_s=e2e_s, h2d=int(h_x0.nbytes + h_u.nbytes + h_abc.nbytes),
-                d2h=int(sum(out[k].nbytes for k in ("xPred", "uPred", "slack", "status", "iters", "resid"))), late=late)
+                d2h=int(sum(out[k].nbytes for k in ("xPred", "uPred", "slack", "status", "iters", "resid"))), late=late, outputs=outputs)
 
 
-def leg_config2(args, rank, world, local, dev, steps=None, with_e2e=True):
+def leg_config2(args, rank, world, local, dev, with_e2e=True):
     """configs[2]: full LMPC steps (K1 -> K2 -> QP<12,48> -> shift), per-instance 5-lap stores."""
     import torch
     import torch.distributed as dist
     from racinglmpc_b200 import workloads, reference_params as rp
     from racinglmpc_b200.controller import BatchedController
     B, N = args.batch, HORIZON
-    steps = steps or args.steps
+    steps = args.steps
     seg = workloads.track_seg_table()      # Map.PointAndTangent[:,3:6] from the reference-pinned fixture
     data = workloads.lmpc_batch(B, seed=2 + rank)
     numSS_it, numSS_Points, _, _, Qts, par = rp.lmpc_params(N)
@@ -420,6 +446,8 @@ def leg_config2(args, rank, world, local, dev, steps=None, with_e2e=True):
         c.sync()
     launches = c.kernel_launches - l0
     torch.cuda.synchronize()
+    # the device-resident step hands its caller the step results and the shifted controller state
+    outputs = dict(c.step_results(), **c.get_state()) if args.dump_outputs else None
     step_ms = [a.elapsed_time(b) for a, b in ev]
     tot = _max_over_ranks(sum(step_ms), dev, world)
     # per-kernel durations (CUDA events between the four launches of one step, L2 flushed, median of a few steps)
@@ -454,7 +482,7 @@ def leg_config2(args, rank, world, local, dev, steps=None, with_e2e=True):
     late = c.late_accepts
     c.close()
     return dict(B=B, steps=steps, total_ms=tot, launches=int(launches), kernel_ms=[float(v) for v in kms], ok=ok, iters=res["iters"],
-                rows_model=rows_model, rows_ss=rows_ss, e2e=e2e, data=data, late=late)
+                rows_model=rows_model, rows_ss=rows_ss, e2e=e2e, data=data, late=late, outputs=outputs)
 
 
 def config2_block(r, world, probe, peaks):
@@ -538,9 +566,11 @@ def run_gpu(args):
                                  "algorithmic_bytes_per_solve": ALGO_BYTES_PER_SOLVE,
                                  "peak_source": "measured (MEASURED_PEAKS.json hbm_gbs)" if "hbm_gbs" in peaks else "fallback 6.65 TB/s"}},
         }
+    dumps = {"config1": r1["outputs"]}
     # ---- the other BASELINE configurations, same process, all ranks (weak scaling: every rank its own batch)
     if not args.headline_only:
-        r2 = leg_config2(args, rank, world, local, dev, steps=max(3, min(args.steps, 10)))
+        r2 = leg_config2(args, rank, world, local, dev)
+        dumps["config2"] = r2["outputs"]
         from benchmarks import rollout_mc
         r3 = rollout_mc.run(batch=args.rollout_batch, laps=3, mode="pooled", share=2, local=local)
         if rank == 0:
@@ -550,6 +580,8 @@ def run_gpu(args):
     if rank == 0:
         if not args.no_cpu_baseline and world == 1:       # the CPU leg is measured at N = 1 only (rank 0 has the host to itself)
             line["cpu_baseline"] = cpu_baseline_block(cpu_arm(oracle_problem_set(CPU_SAMPLE)))
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, dumps)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -582,6 +614,8 @@ def run_lmpc_steps(args):
                 "roofline": dict(blk["kernels"]["ftocp_kernel<12,48,2,4>"]["roofline"], kernel="ftocp_kernel<12,48,2,4>")}
         if not args.no_cpu_baseline:
             line["cpu_baseline"] = lmpc_cpu_baseline(r["data"])
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"config2": r["outputs"]})
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -650,7 +684,10 @@ def main():
                          "1 = configs[1] only; 2 = batch=4096 full LMPC steps as its own line; 3 = Monte-Carlo rollouts as its own line")
     ap.add_argument("--batch", type=int, default=BATCH)
     ap.add_argument("--rollout-batch", type=int, default=8192, help="controllers per GPU of the configs[3] leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step of configs[1] / configs[2] returned as DIR/*.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.config == 3):
+        ap.error("--dump-outputs covers the configs[1] and configs[2] legs of the GPU implementation")
     cpu_threads()                 # read the affinity mask before any OpenMP runtime pins this thread
     if args.config == 1:
         args.headline_only = True

@@ -1,6 +1,5 @@
 import os
 import sys
-import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -15,7 +14,8 @@ def pytest_configure(config):
 
 @pytest.fixture(scope="session")
 def gold():
-    return np.load(os.path.join(ROOT, "tests", "golden", "reference_golden.npz"))
+    from golden_file import GoldenFile
+    return GoldenFile(os.path.join(ROOT, "tests", "golden", "reference_golden.npz"))
 
 
 @pytest.fixture(scope="session")

@@ -26,11 +26,13 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests", "support"))
 REF = "/root/reference/src"
 OUT = os.path.dirname(os.path.abspath(__file__))
 
 from oracle import osqp_port, ftocp, vehicle, ltv_model   # noqa: E402
 from oracle.track import TrackTable                       # noqa: E402
+import golden_file                                        # noqa: E402
 
 
 # ------------------------------------------------------------------ stubs
@@ -325,7 +327,7 @@ def main():
     gold["lmpc_lap_lengths"] = np.array(lap_lengths)
     print("LMPC lock-step laps 4-6: max |diff| =", worst)
 
-    np.savez_compressed(os.path.join(OUT, "reference_golden.npz"), **gold)
+    golden_file.save(os.path.join(OUT, "reference_golden.npz"), gold)
     print("wrote", os.path.join(OUT, "reference_golden.npz"), len(gold), "arrays")
 
 
